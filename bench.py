@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- edited images/sec at 512x512 / 50-step DDIM / CFG (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one complete CFG DDIM sampling run (``DDIMSampler.sample``: 50 UNet evaluations on the
@@ -59,7 +59,12 @@ def parse():
     ap.add_argument("--extra", default="C2,C3,C4,dpm20,pipeline", help="comma list of extra legs to run")
     ap.add_argument("--c2-total", type=int, default=64, help="configs[2]: requests summed over all GPUs")
     ap.add_argument("--c2-chunk", type=int, default=16, help="configs[2]: requests per sampling call on one GPU")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed sampling call returned (rank 0) as DIR/<name>.npy, float32")
+    args = ap.parse_args()
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs needs --steps >= 1")
+    return args
 
 
 # ---- clocks sampler (nvidia-smi during the timed region) ------------------------------------------
@@ -249,6 +254,29 @@ def conds(devt):
     return cond, uncond
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, last):
+    """Writes what ``DDIMSampler.sample`` returned in the final timed call: ``samples`` [B, 4, h, h] and the logged
+    ``x_inter_<i>`` / ``pred_x0_<i>`` latents, float32 .npy.  Inputs are seeded, so two builds can be compared file by file.
+    Should the arrays pass DUMP_BYTES in all, each is cut to the same seeded sample of its flattened elements."""
+    import numpy as np
+    import torch
+    arrays = {"samples": last["samples"]}
+    for key in ("x_inter", "pred_x0"):
+        arrays.update({f"{key}_{i}": t for i, t in enumerate(last["intermediates"][key])})
+    arrays = {k: v.detach().float().cpu() for k, v in arrays.items()}
+    budget = DUMP_BYTES - 4096 * len(arrays)           # room for the .npy headers
+    keep = min(1.0, budget / sum(4 * a.numel() for a in arrays.values()))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if keep < 1.0:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:int(keep * a.numel())]
+            a = a.reshape(-1)[idx.sort().values]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy())
+
+
 def main():
     args = parse()
     rank = int(os.environ.get("RANK", "0"))
@@ -338,6 +366,14 @@ def main():
                        unconditional_conditioning=u_)
     if rank == 0:
         clocks.start()
+    last = {}
+    if args.dump_outputs:                 # keep what each sampler call returns; without the flag the timed path is untouched
+        sample = sampler.sample
+
+        def recorded_sample(*a, **kw):
+            last["samples"], last["intermediates"] = res = sample(*a, **kw)
+            return res
+        sampler.sample = recorded_sample
     if os.environ.get("ANYSD_NCU"):      # ncu --profile-from-start off: launch list of the timed region only
         torch.cuda.cudart().cudaProfilerStart()
     t_res, t_e2e, launches, h2d, d2h = sampling_leg(sampler, [host], S, h, args.scale, 0, args.steps)
@@ -345,6 +381,8 @@ def main():
     if os.environ.get("ANYSD_NCU"):
         torch.cuda.cudart().cudaProfilerStop()
     clk = clocks.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
 
     imgs = B * world * args.steps
     value, e2e = imgs / t_res, imgs / t_e2e

@@ -70,8 +70,11 @@ def main():
         out, inter = sampler.sample(S, 1, (4, h, h), {"c_concat": [c_cat], "c_crossattn": [c_txt]}, verbose=False, x_T=x_T,
                                     eta=0.0, unconditional_guidance_scale=scale, log_every_t=log_every_t,
                                     unconditional_conditioning={"c_concat": [c_cat], "c_crossattn": [u_txt]})
-        extra = {"pred_x0": torch.stack(inter["pred_x0"]).numpy()} if h <= 64 else {}      # (96x96: keep the fixture ~1 MB)
-        np.savez(os.path.join(HERE, f"{name}.npz"), final=out.numpy(), x_inter=torch.stack(inter["x_inter"]).numpy(),
+        x_inter = torch.stack(inter["x_inter"]).numpy()
+        # 96x96: keep the fixture under 1 MB -- no pred_x0, and x_inter (printed along the trajectory, never asserted on) in
+        # fp16; the asserted final latent stays fp32
+        extra = {"pred_x0": torch.stack(inter["pred_x0"]).numpy()} if h <= 64 else {}
+        np.savez(os.path.join(HERE, f"{name}.npz"), final=out.numpy(), x_inter=x_inter if h <= 64 else x_inter.astype(np.float16),
                  S=S, seed=seed, scale=scale, log_every_t=log_every_t, in_sum=checksum(x_T, c_cat, c_txt, u_txt), wsum=wsum, **extra)
         print(f"{name} done in {time.time() - t0:.0f} s", flush=True)
 

@@ -644,3 +644,31 @@ def test_anysd_sampling_shared_halves_and_kept_kv_bit_identical(monkeypatch):
     smp.sample(5, B, (4, 16, 16), cond, verbose=False, x_T=x_T, eta=0.0, unconditional_guidance_scale=7.5,
                unconditional_conditioning={**unc, "c_task": torch.tensor([1, 1, 1]).cuda()})
     assert next(iter(smp._graphs.values())).shared is False
+
+
+def test_bench_dump_outputs_repeatable(tmp_path):
+    """``bench.py --dump-outputs`` on a small workload, twice with different ``--steps``: the timed region runs ``--steps`` passes
+    (its launch count scales with it), and the samples and intermediates of its last call are the same file for file -- the
+    seeded inputs and weights do not depend on the run."""
+    import subprocess
+    import sys
+    root = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
+    runs = {}
+    for steps in (2, 3):
+        out = tmp_path / f"steps{steps}"
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+                            "--batch", "2", "--latent", "32", "--ddim-steps", "5", "--skip-cpu", "--skip-roofline", "--skip-extra",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-2000:]
+        lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
+        assert len(lines) == 1, lines
+        runs[steps] = (json.loads(lines[0]), {f[:-4]: np.load(out / f) for f in os.listdir(out)})
+    (d2, a), (d3, b) = runs[2], runs[3]
+    assert d2["steps"] == 2 and d3["steps"] == 3 and d2["gpu_launches"] > 0
+    assert d2["gpu_launches"] * 3 == d3["gpu_launches"] * 2
+    assert set(a) == {"samples", "x_inter_0", "x_inter_1", "x_inter_2", "pred_x0_0", "pred_x0_1", "pred_x0_2"} == set(b)
+    assert a["samples"].shape == (2, 4, 32, 32) and a["samples"].dtype == np.float32
+    assert np.isfinite(a["samples"]).all() and np.array_equal(a["samples"], a["x_inter_2"])
+    assert rel(torch.from_numpy(a["samples"]), torch.from_numpy(a["x_inter_0"])) > 0.05
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k

@@ -142,6 +142,29 @@ def test_bench_reference_arm_contract(tmp_path):
     assert cb["kind"] == ("reference" if ref_import.available() else "port")
 
 
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """``bench.py --dump-outputs``: the samples and every logged intermediate of the final sampler call as float32 .npy, whole
+    while they fit the byte budget, else each cut to the same seeded sample of its elements, identically from call to call."""
+    import bench
+    gen = torch.Generator().manual_seed(0)
+    lat = lambda: torch.randn(2, 4, 8, 8, generator=gen, dtype=torch.float64)
+    last = {"samples": lat(), "intermediates": {"x_inter": [lat(), lat()], "pred_x0": [lat(), lat()]}}
+    names = {"samples", "x_inter_0", "x_inter_1", "pred_x0_0", "pred_x0_1"}
+    bench.dump_outputs(str(tmp_path / "full"), last)
+    assert {f[:-4] for f in os.listdir(tmp_path / "full")} == names
+    got = np.load(tmp_path / "full" / "samples.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, last["samples"].float().numpy())
+    assert np.array_equal(np.load(tmp_path / "full" / "pred_x0_1.npy"), last["intermediates"]["pred_x0"][1].float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 5 * 4096 + 5 * 4 * 256)   # room for half of each array
+    for d in ("cut_a", "cut_b"):
+        bench.dump_outputs(str(tmp_path / d), last)
+    assert sum(os.path.getsize(tmp_path / "cut_a" / f) for f in os.listdir(tmp_path / "cut_a")) <= bench.DUMP_BYTES
+    for n in names:
+        a, b = np.load(tmp_path / "cut_a" / f"{n}.npy"), np.load(tmp_path / "cut_b" / f"{n}.npy")
+        assert a.dtype == np.float32 and a.shape == (256,) and np.array_equal(a, b)
+        assert np.isin(a, np.load(tmp_path / "full" / f"{n}.npy")).all()
+
+
 def test_no_cpu_fallback():
     """Without a CUDA device the product path must fail loudly, never fall back."""
     from anyedit_b200 import ops
