@@ -90,6 +90,7 @@ SIGNATURES = {
     "anysd_gemm_f16": (_I, [C.POINTER(GemmParams), _VP]),
     "anysd_gemm_stats_slabs": (_I, [C.POINTER(GemmParams)]),
     "anysd_gemm_splitk_workspace_bytes": (_SZ, [C.POINTER(GemmParams)]),
+    "anysd_gemm_schedule": (_I, [C.POINTER(GemmParams)] + [C.POINTER(C.c_int)] * 6),
     "anysd_groupnorm_apply_nhwc_f16": (_I, [_VP, _I, _VP, _I, _VP, _I, _VP, _VP, _VP, _I, _I, _I, _F, _I, _VP, _SZ, _VP]),
     "anysd_attention_f16": (_I, [C.POINTER(AttnParams), _VP]),
     "anysd_cfg_ddim_step_f32": (_I, [_VP, _VP, _VP, _VP, _F, _I, _I, _VP, _VP, _LL, _I, _VP]),

@@ -12,11 +12,14 @@ int launch_gemm_tc5p(const anysd_gemm_params* q, cudaStream_t st);
 bool tc5p_supported(const anysd_gemm_params* q);
 int tc5p_stats_slabs(const anysd_gemm_params* q);
 size_t tc5p_splitk_bytes(const anysd_gemm_params* q);
+int tc5p_schedule(const anysd_gemm_params* q, int* ctas, int* bn, int* splits, int* ext, int* ln);
 }
 
 using namespace anysd;
 
-extern "C" int anysd_gemm_f16(const anysd_gemm_params* p, anysd_stream_t stream) {
+enum { GEMM_MMA = 0, GEMM_TC5 = 1, GEMM_TC5P = 2 };
+
+static int gemm_validate(const anysd_gemm_params* p) {
     ANYSD_REQUIRE(p != nullptr, ANYSD_EINVAL, "gemm: null params");
     ANYSD_REQUIRE(p->A && p->W && p->out, ANYSD_EINVAL, "gemm: null A/W/out");
     ANYSD_REQUIRE(p->M > 0 && p->N > 0 && p->K > 0, ANYSD_EINVAL, "gemm: bad M=%d N=%d K=%d", p->M, p->N, p->K);
@@ -51,6 +54,12 @@ extern "C" int anysd_gemm_f16(const anysd_gemm_params* p, anysd_stream_t stream)
         ANYSD_REQUIRE(p->lda % 8 == 0 && p->lda >= p->K, ANYSD_EINVAL, "gemm: lda=%d must be a multiple of 8 and >= K",
                       p->lda);
     }
+    return ANYSD_OK;
+}
+
+// Kernel selection, shared by the launch and anysd_gemm_schedule: GEMM_MMA / GEMM_TC5 / GEMM_TC5P, or an error code (< 0) when the
+// params ask for something only the persistent kernel can do and it cannot take them.
+static int gemm_kernel(const anysd_gemm_params* p) {
     // Kernel selection.  The persistent tcgen05/TMA kernel (gemm_tc5p.cu) takes every fp16-output contraction
     // whose layout constraints hold: all nn.Linear / 1x1 convs and every 3x3 conv with Cin % 64 == 0 (stride 1|2,
     // upsample through the workspace).  The one-tile-per-CTA tcgen05 kernel (gemm_tc5.cu) takes the fp32-output
@@ -59,14 +68,44 @@ extern "C" int anysd_gemm_f16(const anysd_gemm_params* p, anysd_stream_t stream)
     static const char* force = getenv("ANYSD_GEMM");
     const bool allow_p = !force || !strcmp(force, "tc5p");
     const bool allow_1 = !force || !strcmp(force, "tc5");
-    if (allow_p && tc5p_supported(p)) return launch_gemm_tc5p(p, (cudaStream_t)stream);
+    if (allow_p && tc5p_supported(p)) return GEMM_TC5P;
     ANYSD_REQUIRE(p->row_stats == nullptr && p->ln_stats == nullptr, ANYSD_EUNSUPPORTED,
                   "gemm: LayerNorm fold / row statistics need the persistent tcgen05 path");
     ANYSD_REQUIRE(p->stats == nullptr, ANYSD_EUNSUPPORTED, "gemm: output statistics need the persistent tcgen05 path");
     ANYSD_REQUIRE(!(p->conv && p->conv_pad), ANYSD_EUNSUPPORTED,
                   "conv3x3 with right/bottom padding needs the persistent tcgen05 path (fp16 output, Cin %% 64 == 0)");
-    if ((allow_1 || (force && !strcmp(force, "tc5p"))) && tc5_supported(p)) return launch_gemm_tc5(p, (cudaStream_t)stream);
-    return launch_gemm_mma(p, (cudaStream_t)stream);
+    if ((allow_1 || (force && !strcmp(force, "tc5p"))) && tc5_supported(p)) return GEMM_TC5;
+    return GEMM_MMA;
+}
+
+extern "C" int anysd_gemm_f16(const anysd_gemm_params* p, anysd_stream_t stream) {
+    const int rc = gemm_validate(p);
+    if (rc != ANYSD_OK) return rc;
+    switch (const int k = gemm_kernel(p)) {
+        case GEMM_TC5P: return launch_gemm_tc5p(p, (cudaStream_t)stream);
+        case GEMM_TC5: return launch_gemm_tc5(p, (cudaStream_t)stream);
+        case GEMM_MMA: return launch_gemm_mma(p, (cudaStream_t)stream);
+        default: return k;
+    }
+}
+
+extern "C" int anysd_gemm_schedule(const anysd_gemm_params* p, int* kernel, int* ctas, int* bn, int* splits, int* ext, int* ln) {
+    const int rc = gemm_validate(p);
+    if (rc != ANYSD_OK) return rc;
+    const int k = gemm_kernel(p);
+    if (k < 0) return k;
+    int c = 0, w = 0, s = 0, x = 0, l = 0;
+    if (k == GEMM_TC5P) {
+        const int rs = tc5p_schedule(p, &c, &w, &s, &x, &l);
+        if (rs != ANYSD_OK) return rs;
+    }
+    if (kernel) *kernel = k;
+    if (ctas) *ctas = c;
+    if (bn) *bn = w;
+    if (splits) *splits = s;
+    if (ext) *ext = x;
+    if (ln) *ln = l;
+    return ANYSD_OK;
 }
 
 extern "C" int anysd_gemm_stats_slabs(const anysd_gemm_params* p) {

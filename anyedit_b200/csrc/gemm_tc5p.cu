@@ -892,18 +892,22 @@ int tc5p_stats_slabs(const anysd_gemm_params* q) {
 
 static void p_select(const anysd_gemm_params* q, int tiles_m, int num_kb, int* ctas_out, int* bn_out, int* splits_out);
 static size_t p_splitk_bytes(int tiles_m, int N, int ctas, int bn, int splits);
-// scratch the caller should provide for this contraction to run split-K (0: the schedule does not split it)
-size_t tc5p_splitk_bytes(const anysd_gemm_params* q) {
-    int tiles_m, num_kb;
+// 128-row output tiles and 64-wide k-blocks of the contraction
+static void p_tiles(const anysd_gemm_params* q, int* tiles_m, int* num_kb) {
     if (q->conv) {
         int Ho, Wo, BW, BH, NB;
         p_conv_patch(q, &Ho, &Wo, &BW, &BH, &NB);
-        tiles_m = cdiv(Wo, BW) * cdiv(Ho, BH) * cdiv(q->Nimg, NB);
-        num_kb = 9 * (q->Cin / P_BK);
+        *tiles_m = cdiv(Wo, BW) * cdiv(Ho, BH) * cdiv(q->Nimg, NB);
+        *num_kb = 9 * (q->Cin / P_BK);
     } else {
-        tiles_m = cdiv(q->M, P_BM);
-        num_kb = cdiv(q->K, P_BK);
+        *tiles_m = cdiv(q->M, P_BM);
+        *num_kb = cdiv(q->K, P_BK);
     }
+}
+// scratch the caller should provide for this contraction to run split-K (0: the schedule does not split it)
+size_t tc5p_splitk_bytes(const anysd_gemm_params* q) {
+    int tiles_m, num_kb;
+    p_tiles(q, &tiles_m, &num_kb);
     int ctas, bn, splits;
     p_select(q, tiles_m, num_kb, &ctas, &bn, &splits);
     return p_splitk_bytes(tiles_m, q->N, ctas, bn, splits);
@@ -1056,17 +1060,50 @@ static size_t p_splitk_bytes(int tiles_m, int N, int ctas, int bn, int splits) {
     return (size_t)cdiv(tiles_m, ctas) * cdiv(N, bn) * ctas * splits * P_BM * bn * sizeof(float);
 }
 
+// What launch_gemm_tc5p runs for q (also answers anysd_gemm_schedule, so the query cannot drift from the launch): the cost
+// model's choice, unsplit when the caller withholds the split-K scratch; ext = the extended epilogue (GroupNorm statistics,
+// split-K, GELU / QuickGELU), ln = the LayerNorm-fold epilogue (row statistics out or folded LayerNorm in).  Returns ANYSD_OK,
+// or the error the launch would report for an epilogue combination this kernel cannot run.
+int tc5p_schedule(const anysd_gemm_params* q, int* ctas, int* bn, int* splits, int* ext, int* ln) {
+    if (q->stats != nullptr && (tc5p_stats_slabs(q) == 0 || q->stats_images <= 0)) {
+        set_error("gemm: output statistics requested for a shape that cannot produce them (M=%d rows_per_batch=%d conv=%d act=%d); "
+                  "query anysd_gemm_stats_slabs first", q->M, q->rows_per_batch, q->conv, q->act);
+        return ANYSD_EUNSUPPORTED;
+    }
+    *ln = q->row_stats != nullptr || q->ln_stats != nullptr;
+    if (*ln) {
+        const char* why = tc5p_ln_unsupported(q);
+        if (why) {
+            set_error("gemm: LayerNorm fold / row statistics: %s (M=%d N=%d K=%d act=%d)", why, q->M, q->N, q->K, q->act);
+            return ANYSD_EUNSUPPORTED;
+        }
+    }
+    int tiles_m, num_kb;
+    p_tiles(q, &tiles_m, &num_kb);
+    p_select(q, tiles_m, num_kb, ctas, bn, splits);
+    const size_t sk_need = p_splitk_bytes(tiles_m, q->N, *ctas, *bn, *splits);
+    if (*splits > 1 && (q->splitk_workspace == nullptr || q->splitk_workspace_bytes < sk_need || q->splitk_counters == nullptr ||
+                        (size_t)cdiv(tiles_m, *ctas) * cdiv(q->N, *bn) * *ctas * 8 * sizeof(unsigned int) > q->splitk_counters_bytes)) {
+        *splits = 1;                                  // no scratch from the caller: the plain schedule
+        p_select(q, tiles_m, num_kb, ctas, bn, nullptr);
+    }
+    *ext = q->stats != nullptr || *splits > 1 || q->act >= 3;
+    if (*ln && *ext) {
+        set_error("gemm: LayerNorm fold / row statistics cannot be combined with GroupNorm statistics, split-K or GELU epilogues");
+        return ANYSD_EUNSUPPORTED;
+    }
+    return ANYSD_OK;
+}
+
 int launch_gemm_tc5p(const anysd_gemm_params* q, cudaStream_t st) {
+    int ctas, bn, splits, ext, ln;
+    const int rc = tc5p_schedule(q, &ctas, &bn, &splits, &ext, &ln);
+    if (rc != ANYSD_OK) return rc;
     PArgs a;
     a.stats = nullptr;
     a.stats_hw = a.stats_spi = a.stats_nimg = 0;
     if (q->stats != nullptr) {
         a.stats_spi = tc5p_stats_slabs(q);
-        if (a.stats_spi == 0 || q->stats_images <= 0) {
-            set_error("gemm: output statistics requested for a shape that cannot produce them (M=%d rows_per_batch=%d conv=%d act=%d); "
-                      "query anysd_gemm_stats_slabs first", q->M, q->rows_per_batch, q->conv, q->act);
-            return ANYSD_EUNSUPPORTED;
-        }
         a.stats = q->stats;
         a.stats_hw = q->rows_per_batch;
         a.stats_nimg = q->stats_images;
@@ -1077,14 +1114,6 @@ int launch_gemm_tc5p(const anysd_gemm_params* q, cudaStream_t st) {
     a.ln_slabs = q->K / 64;
     a.ln_eps = q->ln_eps;
     a.ln_inv_k = 1.0f / (float)q->K;
-    const bool ln = q->row_stats != nullptr || q->ln_stats != nullptr;
-    if (ln) {
-        const char* why = tc5p_ln_unsupported(q);
-        if (why) {
-            set_error("gemm: LayerNorm fold / row statistics: %s (M=%d N=%d K=%d act=%d)", why, q->M, q->N, q->K, q->act);
-            return ANYSD_EUNSUPPORTED;
-        }
-    }
     a.bias = q->bias;
     a.rowadd = q->rowadd;
     a.M = q->M;
@@ -1134,14 +1163,6 @@ int launch_gemm_tc5p(const anysd_gemm_params* q, cudaStream_t st) {
         ok = ok && p_map_2d(&tmO, q->out, (uint64_t)n_out, (uint64_t)q->M, (uint64_t)q->ldo, P_SUB, 32);
         if (q->residual) ok = ok && p_map_2d(&tmR, q->residual, (uint64_t)n_out, (uint64_t)q->M, (uint64_t)q->ldr, P_SUB, 32);
     }
-    int ctas = 1, bn = 256, splits = 1;
-    p_select(q, a.tiles_m, a.num_kb, &ctas, &bn, &splits);
-    const size_t sk_need = p_splitk_bytes(a.tiles_m, q->N, ctas, bn, splits);
-    if (splits > 1 && (q->splitk_workspace == nullptr || q->splitk_workspace_bytes < sk_need || q->splitk_counters == nullptr ||
-                       (size_t)cdiv(a.tiles_m, ctas) * cdiv(q->N, bn) * ctas * 8 * sizeof(unsigned int) > q->splitk_counters_bytes)) {
-        splits = 1;                                   // no scratch from the caller: the plain schedule
-        p_select(q, a.tiles_m, a.num_kb, &ctas, &bn, nullptr);
-    }
     a.bn = bn;
     a.tiles_n = cdiv(q->N, bn);
     a.stage_tx = P_A_BYTES + (bn / ctas) * P_BK * 2;
@@ -1157,12 +1178,7 @@ int launch_gemm_tc5p(const anysd_gemm_params* q, cudaStream_t st) {
     a.num_units = a.num_tiles * splits;
     a.sk_ws = (float*)q->splitk_workspace;
     a.sk_cnt = (unsigned int*)q->splitk_counters;
-    const bool ext = a.stats != nullptr || a.splits > 1 || a.act >= 3;
     if (ln) {
-        if (ext) {
-            set_error("gemm: LayerNorm fold / row statistics cannot be combined with GroupNorm statistics, split-K or GELU epilogues");
-            return ANYSD_EUNSUPPORTED;
-        }
         return ctas == 2 ? p_launch<false, 2, false, true>(tmA, tmB, tmO, tmR, a, st) : p_launch<false, 1, false, true>(tmA, tmB, tmO, tmR, a, st);
     }
     if (ext) {

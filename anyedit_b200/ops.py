@@ -241,6 +241,17 @@ def _want_splitk(p, dev):
     return ws
 
 
+SCHEDULE_KEYS = ("kernel", "ctas", "bn", "splits", "ext", "ln")
+
+
+def _fill_schedule(p, schedule):
+    """schedule.update(anysd_gemm_schedule(p)): the kernel (0 mma.sync, 1 tcgen05, 2 persistent tcgen05) and, for the
+    persistent kernel, the CTAs per tile, the tile width, the K split and the epilogue variant these exact params launch."""
+    vals = [C.c_int() for _ in SCHEDULE_KEYS]
+    _lib.check(_lib.load().anysd_gemm_schedule(C.byref(p), *[C.byref(v) for v in vals]), "gemm_schedule")
+    schedule.update(zip(SCHEDULE_KEYS, (v.value for v in vals)))
+
+
 def row_stats_buffer(M, C, device):
     """fp32 [C / 64, M, 2]: the per-row moments a contraction's epilogue writes for the LayerNorm folded into its consumer."""
     assert C % 64 == 0
@@ -248,12 +259,13 @@ def row_stats_buffer(M, C, device):
 
 
 def gemm(A, W, out, bias=None, rowadd=None, rows_per_batch=0, residual=None, act=0, M=None, K=None, lda=None,
-         N=None, ldw=None, ld_rowadd=None, stats_images=0, row_stats=None, ln=None):
+         N=None, ldw=None, ld_rowadd=None, stats_images=0, row_stats=None, ln=None, schedule=None):
     """out[M, N'] = epilogue(A[M, K] @ W[N, K]^T); see anysd_gemm_params.
     ``stats_images`` > 0 (with ``rows_per_batch`` = rows of one image): also produce the GroupNorm statistics of ``out`` in the
     epilogue; returns a GnStats (None when the shape cannot).
     ``row_stats`` (row_stats_buffer(M, N)): per-row moments of ``out`` for a LayerNorm folded into the consumer.
-    ``ln`` = (row statistics of A, column sums of the gamma-scaled W, eps): LayerNorm(A) @ W^T + b with A un-normalised."""
+    ``ln`` = (row statistics of A, column sums of the gamma-scaled W, eps): LayerNorm(A) @ W^T + b with A un-normalised.
+    ``schedule`` (a dict): filled with what this launch runs (anysd_gemm_schedule, keys SCHEDULE_KEYS)."""
     _cuda(A, W, out)
     p = GemmParams()
     p.A, p.W, p.out = A.data_ptr(), W.data_ptr(), out.data_ptr()
@@ -282,6 +294,8 @@ def gemm(A, W, out, bias=None, rowadd=None, rows_per_batch=0, residual=None, act
         p.ln_stats, p.ln_colsum, p.ln_eps = lst.data_ptr(), lcs.data_ptr(), float(leps)
     st = _want_stats(p, stats_images, out.device) if stats_images > 0 else None
     _sk = _want_splitk(p, out.device) if (row_stats is None and ln is None) else None
+    if schedule is not None:
+        _fill_schedule(p, schedule)
     with _Traced("gemm", 2.0 * p.M * p.N * p.K, f"M={p.M} N={p.N} K={p.K} act={p.act} res={int(residual is not None)}"):
         _lib.check(_lib.load().anysd_gemm_f16(C.byref(p), _stream()), "gemm")
     _count()
@@ -289,9 +303,10 @@ def gemm(A, W, out, bias=None, rowadd=None, rows_per_batch=0, residual=None, act
 
 
 def conv3x3(x, W, out, bias=None, rowadd=None, residual=None, stride=1, upsample=0, ld_rowadd=None,
-            logical_cin=None, logical_cout=None, act=0, pad_rb=False, stats=False):
+            logical_cin=None, logical_cout=None, act=0, pad_rb=False, stats=False, schedule=None):
     """x NHWC fp16 [N,H,W,Cin]; W fp16 [Cout, 9*Cin] ((ky,kx,ci) K order); out [N*Ho*Wo, Cout].
-    pad_rb (stride 2 only): zero padding on the right / bottom instead of all around (first-stage Downsample, model.py:83-85)."""
+    pad_rb (stride 2 only): zero padding on the right / bottom instead of all around (first-stage Downsample, model.py:83-85).
+    ``schedule`` (a dict): filled with what this launch runs (see gemm)."""
     _cuda(x, W, out)
     Nimg, H, Wd, Cin = x.shape
     Hl, Wl = H << upsample, Wd << upsample
@@ -324,6 +339,8 @@ def conv3x3(x, W, out, bias=None, rowadd=None, residual=None, stride=1, upsample
     fl = 2.0 * p.M * (logical_cout or p.N) * 9 * (logical_cin or Cin)
     st = _want_stats(p, Nimg, out.device, reuse=stats) if stats else None
     _sk = _want_splitk(p, out.device)
+    if schedule is not None:
+        _fill_schedule(p, schedule)
     with _Traced("conv3x3", fl, f"N={p.Nimg} {p.H}x{p.Wd} {p.Cin}->{p.N} s={p.stride} up={p.upsample} res={int(residual is not None)}"):
         _lib.check(_lib.load().anysd_gemm_f16(C.byref(p), _stream()), "conv3x3")
     _count()

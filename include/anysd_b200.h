@@ -162,6 +162,12 @@ int anysd_gemm_stats_slabs(const anysd_gemm_params* p);
  * sums are added in split order by whichever unit finishes last.  The result therefore depends neither on the batch nor on the
  * arrival order -- but a caller that withholds the scratch gets the unsplit summation order (differs in fp32 rounding). */
 size_t anysd_gemm_splitk_workspace_bytes(const anysd_gemm_params* p);
+/* What anysd_gemm_f16 would launch for these exact params (same validation, same selection code, the split-K scratch as
+ * attached): kernel 0 mma.sync, 1 tcgen05, 2 persistent tcgen05; for kernel 2 also ctas (1 | 2: CTA pairs), bn (tile width
+ * 64 | 128 | 192 | 256), splits (K split, 1 = unsplit), ext (1 = the extended epilogue: GroupNorm statistics / split-K /
+ * GELU / QuickGELU) and ln (1 = the LayerNorm-fold epilogue: row_stats or ln_stats); all 0 for kernels 0 and 1.  Returns the
+ * error code anysd_gemm_f16 would return, ANYSD_OK otherwise.  Any output pointer may be NULL. */
+int anysd_gemm_schedule(const anysd_gemm_params* p, int* kernel, int* ctas, int* bn, int* splits, int* ext, int* ln);
 
 /* ---- attention ---------------------------------------------------------------------------
  * CrossAttention.forward (attention.py:163-194) / xformers memory_efficient_attention (:233):
